@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — headline benchmark of the hot path (BASELINE.json): secp256r1 prj_pt_mul/s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  Default workload (N = 1) is BASELINE.json
 configs[1]: 2^20 random scalars on the fixed base G of secp256r1 per GPU.  The other configs of BASELINE.json
@@ -24,6 +24,11 @@ Ours arm, per step and per rank (one process per GPU; torchrun for N > 1) — th
 
 Reference arm (--impl reference): the reference's own CPU implementation of the path (oracle/_ref, else the oracle
 port) on all host cores, each step a bounded sample of the same workload; rank 0 only.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the last timed step returned to its caller as float32
+.npy files (inputs are seeded, so two builds run with the same arguments can be compared output for output):
+verdicts.npy (one per item) for the verification workloads; points.npy (affine x || y bytes) and status.npy for the
+scalar multiplications, on a fixed seeded sample of DUMP_ITEMS items whose positions are in sample_index.npy.
 """
 from __future__ import annotations
 
@@ -68,6 +73,8 @@ VERIFY_HASH = "SHA256"
 # 180 GB HBM); secp384r1 keeps to 24 bits (24 GiB; 26 bits would be 90 GiB)
 DEFAULT_COMB = {"SECP256R1": int(os.environ.get("BENCH_COMB_WINDOW", "26")),
                 "SECP384R1": int(os.environ.get("BENCH_COMB_WINDOW_384", "24"))}
+# --dump-outputs keeps the files under 64 MB: 2^16 points of secp521r1 are 132 bytes, 35 MB as float32
+DUMP_ITEMS = 1 << 16
 
 
 def splitmix_bytes(n_bytes: int, tag: int) -> np.ndarray:
@@ -293,6 +300,21 @@ def make_verify_inputs(curve: str, n: int, rank: int, use_gpu: bool = True):
     return {"sigs": sigs, "pubkeys": pubs, "msgs": msgs, "digests_host": dg, "expected": expected, "hlen": hlen}
 
 
+def dump_outputs(path: str, kind: str, results) -> None:
+    """--dump-outputs: the last timed step's results, (verdicts,) or (points, status), as float32 .npy files."""
+    os.makedirs(path, exist_ok=True)
+    save = lambda name, a: np.save(os.path.join(path, name + ".npy"), np.asarray(a).astype(np.float32))
+    if kind == "verify":
+        save("verdicts", results[0])
+        return
+    out, st = results
+    n = out.shape[0]
+    idx = np.sort(np.random.default_rng(SEED).choice(n, size=min(n, DUMP_ITEMS), replace=False))
+    np.save(os.path.join(path, "sample_index.npy"), idx.astype(np.float64))
+    save("points", out[idx])
+    save("status", st[idx])
+
+
 # ------------------------------------------------------------------------------------------------ CPU arms
 
 def ref_lib():
@@ -399,8 +421,10 @@ def run_reference(args, rank: int):
     times = []
     for s in range(args.steps):
         lo = (s * per_step) % max(1, n - per_step + 1)
-        t, k, _ = cpu_run(args.workload, inputs, lo, per_step, threads)
+        t, k, outs = cpu_run(args.workload, inputs, lo, per_step, threads)
         times.append(t)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, kind, outs)
     val = per_step * len(times) / sum(times)
     line = {"impl": "reference", "metric": metric, "value": val, "unit": unit, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1000 * sum(times) / len(times),
@@ -992,6 +1016,7 @@ def main():
                          "pipelined one step behind the kernels; fused-*: stores of the normalisation kernel itself)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the short runs of the other BASELINE.json configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", 0))
@@ -1017,6 +1042,8 @@ def main():
     n = o.n
     p2p = o.p2p_probe() if (world > 1 and o.pg is not None and os.environ.get("BENCH_P2P_PROBE")) else None
     m = o.measure_device(args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, o.kind, o.local_results())
     parity = o.parity()
     gchk = o.gather_checks() if world > 1 else {}
     e2e_steps = max(3, min(args.steps, 10))

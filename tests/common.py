@@ -74,14 +74,95 @@ def oracle_lib() -> ctypes.CDLL:
 
 
 def ref_lib():
-    """The unmodified reference compiled by oracle/Makefile, or None when it is not available (it is built in
-    the container that has /root/reference and travels to the GPU box as a prebuilt .so)."""
+    """The unmodified reference compiled by oracle/Makefile (`make -C oracle ref REF=<its sources>`).  Only the
+    @reference_answer helpers call it, and only while their answers are being recorded."""
     if "ref" not in _cache:
-        if not os.path.exists(REF_SO) and os.path.exists("/root/reference/src/libsig.h"):
-            subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "-j8", "ref"], check=True,
-                           capture_output=True)
-        _cache["ref"] = ctypes.CDLL(REF_SO) if os.path.exists(REF_SO) else None
+        if not os.path.exists(REF_SO):
+            raise RuntimeError(f"{REF_SO} is missing: build it with `make -C oracle ref REF=<reference sources>`")
+        _cache["ref"] = ctypes.CDLL(REF_SO)
     return _cache["ref"]
+
+
+# The reference's answers to the questions the tests ask it are stored under tests/golden/reference/ (one xz-compressed
+# .npz per test module), keyed by the helper's name and a digest of its arguments, so that the comparisons run on any machine.
+# RECORD_REFERENCE=1 asks the compiled reference instead and stores its answers (tests/golden/record_reference.sh).
+REFERENCE_ANSWERS = os.path.join(GOLDEN, "reference")
+RECORDING = os.environ.get("RECORD_REFERENCE") == "1"
+_answers = {}
+
+
+def _digest_args(h, a):
+    if isinstance(a, np.ndarray):
+        a = np.ascontiguousarray(a)
+        h.update(b"A%s%r" % (a.dtype.str.encode(), a.shape))
+        h.update(a.tobytes())
+    elif isinstance(a, (bytes, bytearray)):
+        h.update(b"B%d:" % len(a))
+        h.update(bytes(a))
+    elif isinstance(a, (list, tuple)):
+        h.update(b"L%d:" % len(a))
+        for x in a:
+            _digest_args(h, x)
+    elif a is None or isinstance(a, (str, int, np.integer)):
+        h.update(b"S%r;" % (a if a is None or isinstance(a, str) else int(a),))
+    else:
+        raise TypeError(f"cannot key a reference answer on {type(a)}")
+
+
+def _answer_file(module: str):
+    if module not in _answers:
+        import io
+        import lzma
+        path = os.path.join(REFERENCE_ANSWERS, module + ".npz.xz")
+        stored = {}
+        if os.path.exists(path):
+            with lzma.open(path) as f, np.load(io.BytesIO(f.read())) as z:
+                stored = {k: z[k] for k in z.files}
+        _answers[module] = stored
+    return _answers[module]
+
+
+def _save_answers():
+    import io
+    import lzma
+    os.makedirs(REFERENCE_ANSWERS, exist_ok=True)
+    for module, stored in _answers.items():
+        buf = io.BytesIO()
+        np.savez(buf, **stored)    # one xz stream: the many small answers share their headers' compression
+        with open(os.path.join(REFERENCE_ANSWERS, module + ".npz.xz"), "wb") as f:
+            f.write(lzma.compress(buf.getvalue(), preset=9 | lzma.PRESET_EXTREME))
+
+
+def reference_answer(fn):
+    """Decorates a helper that asks the compiled reference something: its arguments are arrays, bytes, strings or ints,
+    its result an array or an int, or a tuple of them.  The stored answer for the same arguments is returned; a question
+    without a stored answer fails (its inputs changed: record the answers again)."""
+    import functools
+    import hashlib
+
+    @functools.wraps(fn)
+    def ask(*args):
+        h = hashlib.sha256()
+        _digest_args(h, args)
+        key = f"{fn.__name__}-{h.hexdigest()[:24]}"
+        stored = _answer_file(fn.__module__)
+        if RECORDING:
+            if "save" not in _cache:
+                import atexit
+                _cache["save"] = atexit.register(_save_answers)
+            res = fn(*args)
+            items = res if isinstance(res, tuple) else (res,)
+            stored[key + ".n"] = np.array(len(items) if isinstance(res, tuple) else -1)
+            for i, x in enumerate(items):
+                stored[f"{key}.{i}"] = np.asarray(x)
+        if key + ".n" not in stored:
+            raise AssertionError(f"no stored answer of the reference to {fn.__module__}.{fn.__name__} for these "
+                                 f"arguments: record them again (tests/golden/record_reference.sh)")
+        n = int(stored[key + ".n"])
+        items = [stored[f"{key}.{i}"] for i in range(max(n, 1))]
+        items = [x.item() if x.ndim == 0 else x.copy() for x in items]
+        return tuple(items) if n >= 0 else items[0]
+    return ask
 
 
 def hostsim_lib() -> ctypes.CDLL:
@@ -179,6 +260,12 @@ def oracle_smul(curve: str, scalars: np.ndarray, points=None, nthreads: int = 8,
     rc = fn(curve.encode(), n, _buf(sc), qlen, _buf(pts) if pts is not None else None, _buf(out), _buf(st), nthreads)
     assert rc == 0
     return out, st
+
+
+@reference_answer
+def ref_smul(curve: str, scalars: np.ndarray, points=None):
+    """(out, status) of the compiled reference's prj_pt_mul for the same inputs as oracle_smul."""
+    return oracle_smul(curve, scalars, points, lib=ref_lib())
 
 
 def oracle_verify(curve: str, sigs, pubkeys, digests, hlen: int, nthreads: int = 8) -> np.ndarray:

@@ -48,3 +48,20 @@ def test_other_ranks_of_the_reference_arm_exit_without_work():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
                         "--warmup", "0"], capture_output=True, text=True, timeout=300, env=env, cwd=ROOT)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_reference_arm_dumps_the_last_steps_outputs(tmp_path):
+    """--dump-outputs: float32 / float64 .npy files under 64 MB, identical for two runs with the same arguments."""
+    import numpy as np
+    runs = []
+    for name in ("a", "b"):
+        _ref_line(["--batch-log2", "8", "--dump-outputs", str(tmp_path / name)])
+        files = sorted(os.listdir(tmp_path / name))
+        assert files == ["points.npy", "sample_index.npy", "status.npy"]
+        runs.append({f[:-4]: np.load(tmp_path / name / f) for f in files})
+    a, b = runs
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    assert all(x.dtype in (np.float32, np.float64) for x in a.values())
+    assert a["points"].shape == (256, 64) and a["status"].shape == (256,)
+    assert set(np.unique(a["status"])) <= {0.0, 1.0}
+    assert all((a[f] == b[f]).all() for f in a)

@@ -1,15 +1,15 @@
 """BIP0340 verification (SURVEY.md §8f.4; reference: src/sig/bip0340.c:383-577).
 
 CPU: the oracle port against the reference's own BIP0340 known-answer vectors (tests/golden/bip0340_kat.json, from
-src/tests/bip0340_test_vectors.h) and against the unmodified reference on signatures the reference made; the host
-build of the kernel's algorithm against the oracle.  GPU (`-m gpu`): the C ABI against the oracle / the reference,
-corrupted signatures included."""
+src/tests/bip0340_test_vectors.h) and against the unmodified reference on signatures the reference made (its
+signatures and verdicts are stored under tests/golden/reference/); the host build of the kernel's algorithm against
+the oracle.  GPU (`-m gpu`): the C ABI against the oracle / the reference, corrupted signatures included."""
 import hashlib
 
 import numpy as np
 import pytest
 
-from common import ALL_CURVES, HASHLEN, ORDER, PRIME, golden, hostsim_lib, hx, oracle_lib, random_scalars, ref_lib, rng, _buf
+from common import ALL_CURVES, HASHLEN, ORDER, PRIME, golden, hostsim_lib, hx, oracle_lib, random_scalars, ref_lib, reference_answer, rng, _buf
 
 HASH = {"SHA256": hashlib.sha256, "SHA384": hashlib.sha384, "SHA512": hashlib.sha512}
 TAG = b"BIP0340/challenge"
@@ -38,6 +38,7 @@ def pack(msgs):
     return blob, off
 
 
+@reference_answer
 def ref_sign(curve, hash_name, privs, msgs):
     ref = ref_lib()
     _, plen, qlen = ALL_CURVES[curve]
@@ -51,6 +52,7 @@ def ref_sign(curve, hash_name, privs, msgs):
     return sigs, pubs
 
 
+@reference_answer
 def ref_verify(curve, hash_name, sigs, pubs, msgs):
     ref = ref_lib()
     n = sigs.shape[0]
@@ -59,6 +61,14 @@ def ref_verify(curve, hash_name, sigs, pubs, msgs):
     assert ref.ref_bip0340_verify_batch(curve.encode(), hash_name.encode(), n, _buf(sigs), _buf(pubs), _buf(blob),
                                         _buf(off), _buf(v), 8) == 0
     return v
+
+
+@reference_answer
+def ref_verify_batch_all(curve, hash_name, sigs, pubs, msgs, scratch):
+    """ec_verify_batch(..., BIP0340, ...) of the reference, with or without a scratch pad: 0 / -1."""
+    blob, off = pack(msgs)
+    return ref_lib().ref_bip0340_verify_batch_all(curve.encode(), hash_name.encode(), sigs.shape[0], _buf(sigs),
+                                                  _buf(pubs), _buf(blob), _buf(off), scratch)
 
 
 def workload(curve, n, tag, hash_name="SHA256"):
@@ -106,8 +116,6 @@ def test_oracle_against_reference_kats():
 @pytest.mark.parametrize("curve,hash_name", [("SECP256K1", "SHA256"), ("SECP256R1", "SHA512"), ("FRP256V1", "SHA256"),
                                              ("SECP384R1", "SHA384"), ("SECP192R1", "SHA256")])
 def test_oracle_and_host_algorithm_against_reference(curve, hash_name):
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     sigs, pubs, dg, hlen, want = workload(curve, 28, 8100, hash_name)
     assert (oracle_bip_verify(curve, sigs, pubs, dg, hlen) == want).all()
     got = np.zeros(len(want), np.int8)
@@ -120,8 +128,6 @@ def test_oracle_and_host_algorithm_against_reference(curve, hash_name):
 @pytest.mark.parametrize("curve", list(ALL_CURVES))
 def test_gpu_bip0340_verify(curve):
     import libecc_b200
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     _, plen, qlen = ALL_CURVES[curve]
     eng = libecc_b200.Engine(curve, comb_window=8)
     for tag, hname in ((8300, "SHA256"), (8400, "SHA512")):
@@ -139,8 +145,6 @@ def test_gpu_bip0340_verify(curve):
 def test_gpu_bip0340_large_batch():
     """2^16 signatures through the chunked host pipeline: tiled reference-made signatures, every 4th corrupted."""
     import libecc_b200
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     curve = "SECP256K1"
     sigs, pubs, dg, hlen, want = workload(curve, 256, 8500)
     reps = 1 << 8

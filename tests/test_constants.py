@@ -1,12 +1,14 @@
 """Device constants (tools/gen_curve_constants.py -> libecc_b200/csrc/curve_constants.inc) against the reference's
-own curve parameters (read through ref_curve_info from src/curves/known/ec_params_*.h) and plain integers."""
+own curve parameters (read through ref_curve_info from src/curves/known/ec_params_*.h, stored under tests/golden/reference/)
+and plain integers."""
 import ctypes
 import os
 import re
 
+import numpy as np
 import pytest
 
-from common import ALL_CURVES, CURVES, ORDER, PRIME, ROOT, ref_lib
+from common import ALL_CURVES, CURVES, ORDER, PRIME, ROOT, ref_lib, reference_answer
 
 
 def parse_inc():
@@ -26,6 +28,15 @@ def parse_inc():
     return out
 
 
+@reference_answer
+def ref_curve_info(curve):
+    """plen, qlen and the big-endian p, q, a, b, gx, gy of the reference's curve parameters."""
+    plen, qlen = ctypes.c_uint32(), ctypes.c_uint32()
+    bufs = [ctypes.create_string_buffer(66) for _ in range(6)]
+    assert ref_lib().ref_curve_info(curve.encode(), ctypes.byref(plen), ctypes.byref(qlen), *bufs) == 0
+    return (plen.value, qlen.value) + tuple(np.frombuffer(x.raw[: plen.value], np.uint8) for x in bufs)
+
+
 @pytest.mark.parametrize("curve", list(ALL_CURVES))
 def test_generated_constants(curve):
     inc = parse_inc()
@@ -43,12 +54,7 @@ def test_generated_constants(curve):
     b = c["B_MONT"] * pow(R, -1, p) % p
     a = c["A_MONT"] * pow(R, -1, p) % p
     assert (gy * gy - (gx ** 3 + a * gx + b)) % p == 0
-    ref = ref_lib()
-    if ref is None:
-        pytest.skip("compiled reference not available")
-    plen, qlen = ctypes.c_uint32(), ctypes.c_uint32()
-    bufs = [ctypes.create_string_buffer(66) for _ in range(6)]
-    assert ref.ref_curve_info(curve.encode(), ctypes.byref(plen), ctypes.byref(qlen), *bufs) == 0
-    rp, rq, ra, rb, rgx, rgy = [int.from_bytes(x.raw[: plen.value], "big") for x in bufs]
+    plen, qlen, *bufs = ref_curve_info(curve)
+    rp, rq, ra, rb, rgx, rgy = [int.from_bytes(x.tobytes(), "big") for x in bufs]
     assert (rp, rq, rgx, rgy, rb, ra) == (p, q, gx, gy, b, a)
-    assert (plen.value, qlen.value) == ALL_CURVES[curve][1:]
+    assert (plen, qlen) == ALL_CURVES[curve][1:]

@@ -1,14 +1,15 @@
 """include/libecc_b200_dropin.h mirrors the reference's struct layout: compile a probe against OUR header and compare
-every sizeof/offsetof with the same facts taken from the reference's own headers (oracle/ref_shim.c: ref_abi_facts).
+every sizeof/offsetof with the same facts taken from the reference's own headers (oracle/ref_shim.c: ref_abi_facts,
+stored under tests/golden/reference/).
 Also checks the magic-word constants the drop-in writes."""
 import ctypes
 import os
 import subprocess
 import tempfile
 
-import pytest
+import numpy as np
 
-from common import ROOT, ref_lib
+from common import ROOT, ref_lib, reference_answer
 
 PROBE = r"""
 #include <stddef.h>
@@ -35,19 +36,21 @@ int main(void) {
 """
 
 
+@reference_answer
+def ref_abi_facts():
+    buf = (ctypes.c_uint64 * 64)()
+    k = ref_lib().ref_abi_facts(buf, 64)
+    return np.array(buf[:k], np.uint64)
+
+
 def test_struct_layout_matches_reference():
-    ref = ref_lib()
-    if ref is None:
-        pytest.skip("compiled reference not available")
     with tempfile.TemporaryDirectory() as td:
         src = os.path.join(td, "probe.c")
         open(src, "w").write(PROBE)
         exe = os.path.join(td, "probe")
         subprocess.run(["gcc", "-I", os.path.join(ROOT, "include"), src, "-o", exe], check=True)
         ours = [int(x) for x in subprocess.run([exe], check=True, capture_output=True, text=True).stdout.split()]
-    buf = (ctypes.c_uint64 * 64)()
-    k = ref.ref_abi_facts(buf, 64)
-    facts = list(buf[:k])
+    facts = [int(x) for x in ref_abi_facts()]
     # ref_abi_facts order: nn(3) fp(3) prj_pt(5) fp_ctx(6) crv(5) ec_params(7) ec_pub_key(4) NN_MAX_WORD_LEN
     ref_struct = facts[:22]
     ref_pub = facts[29:33]

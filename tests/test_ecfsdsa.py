@@ -1,15 +1,16 @@
 """ECFSDSA verification (SURVEY.md §8f.4; reference: src/sig/ecfsdsa.c:416-610).
 
 CPU: the oracle port against the reference's own ECFSDSA known-answer vectors (tests/golden/ecfsdsa_kat.json) and
-against the unmodified reference on signatures the reference made; the host build of the kernel's algorithm against
-the oracle.  GPU (`-m gpu`): the C ABI against the oracle / the reference, corrupted signatures included."""
+against the unmodified reference on signatures the reference made (its signatures and verdicts are stored under
+tests/golden/reference/); the host build of the kernel's algorithm against the oracle.  GPU (`-m gpu`): the C ABI
+against the oracle / the reference, corrupted signatures included."""
 import ctypes
 import hashlib
 
 import numpy as np
 import pytest
 
-from common import ALL_CURVES, HASHLEN, ORDER, PRIME, golden, hostsim_lib, hx, oracle_lib, random_scalars, ref_lib, rng, _buf
+from common import ALL_CURVES, HASHLEN, ORDER, PRIME, golden, hostsim_lib, hx, oracle_lib, random_scalars, ref_lib, reference_answer, rng, _buf
 
 HASH = {"SHA224": hashlib.sha224, "SHA256": hashlib.sha256, "SHA384": hashlib.sha384, "SHA512": hashlib.sha512}
 
@@ -26,7 +27,16 @@ def oracle_fs_verify(curve, sigs, pubs, digests, hlen):
 
 
 def ref_sign(curve, hash_name, privs, msgs):
-    """Signatures and public keys made by the unmodified reference (random nonces)."""
+    """Signatures and public keys made by the unmodified reference (random nonces), and the packed messages."""
+    n = len(msgs)
+    blob = np.frombuffer(b"".join(msgs), dtype=np.uint8).copy()
+    off = np.zeros(n + 1, dtype=np.uint64)
+    off[1:] = np.cumsum([len(m) for m in msgs])
+    return ref_sign_raw(curve, hash_name, privs, msgs) + (blob, off)
+
+
+@reference_answer
+def ref_sign_raw(curve, hash_name, privs, msgs):
     ref = ref_lib()
     _, plen, qlen = ALL_CURVES[curve]
     n = len(msgs)
@@ -38,9 +48,10 @@ def ref_sign(curve, hash_name, privs, msgs):
     st = np.zeros(n, np.int8)
     assert ref.ref_ecfsdsa_sign_batch(curve.encode(), hash_name.encode(), n, _buf(privs), _buf(blob), _buf(off),
                                       _buf(sigs), _buf(pubs), _buf(st), 8) == 0 and (st == 0).all()
-    return sigs, pubs, blob, off
+    return sigs, pubs
 
 
+@reference_answer
 def ref_verify(curve, hash_name, sigs, pubs, blob, off):
     ref = ref_lib()
     n = sigs.shape[0]
@@ -48,6 +59,13 @@ def ref_verify(curve, hash_name, sigs, pubs, blob, off):
     assert ref.ref_ecfsdsa_verify_batch(curve.encode(), hash_name.encode(), n, _buf(sigs), _buf(pubs), _buf(blob),
                                         _buf(off), _buf(v), 8) == 0
     return v
+
+
+@reference_answer
+def ref_verify_batch_all(curve, hash_name, sigs, pubs, blob, off):
+    """ec_verify_batch(..., ECFSDSA, ...) of the reference without a scratch pad: 0 / -1."""
+    return ref_lib().ref_ecfsdsa_verify_batch_all(curve.encode(), hash_name.encode(), sigs.shape[0], _buf(sigs), _buf(pubs),
+                                                  _buf(blob), _buf(off), 0)
 
 
 def workload(curve, n, tag, hash_name=None):
@@ -95,8 +113,6 @@ def test_oracle_against_reference_kats():
                                              ("SECP192R1", "SHA512")])
 def test_oracle_and_host_algorithm_against_reference(curve, hash_name):
     """Digests longer than the order (SHA-512 on P-256, SHA-256 on P-224) exercise the full-digest reduction."""
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     sigs, pubs, dg, hlen, want = workload(curve, 24, 7100, hash_name)
     assert (oracle_fs_verify(curve, sigs, pubs, dg, hlen) == want).all()
     lib = hostsim_lib()
@@ -109,17 +125,13 @@ def test_oracle_and_host_algorithm_against_reference(curve, hash_name):
 def test_reference_batch_entry_point_agrees_on_valid_batches():
     """ec_verify_batch(…, ECFSDSA, …) of the reference (no scratch pad) returns 0 for an all-valid batch and -1 once a
     signature is corrupted — the aggregate of the per-item verdicts this engine reports."""
-    ref = ref_lib()
-    if ref is None:
-        pytest.skip("compiled reference not available")
     curve, hash_name = "FRP256V1", "SHA256"
     privs = random_scalars(curve, 6, tag=7201)
     msgs = [b"batch message %d" % i for i in range(6)]
     sigs, pubs, blob, off = ref_sign(curve, hash_name, privs, msgs)
-    args = (curve.encode(), hash_name.encode(), 6, _buf(sigs), _buf(pubs), _buf(blob), _buf(off))
-    assert ref.ref_ecfsdsa_verify_batch_all(*args, 0) == 0
+    assert ref_verify_batch_all(curve, hash_name, sigs, pubs, blob, off) == 0
     sigs[2, -1] ^= 1
-    assert ref.ref_ecfsdsa_verify_batch_all(*args, 0) == -1
+    assert ref_verify_batch_all(curve, hash_name, sigs, pubs, blob, off) == -1
     assert list(ref_verify(curve, hash_name, sigs, pubs, blob, off)) == [0, 0, -1, 0, 0, 0]
 
 
@@ -127,8 +139,6 @@ def test_reference_batch_entry_point_agrees_on_valid_batches():
 @pytest.mark.parametrize("curve", list(ALL_CURVES))
 def test_gpu_ecfsdsa_verify(curve):
     import libecc_b200
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     eng = libecc_b200.Engine(curve, comb_window=8)
     for tag, hname in ((7300, None), (7400, "SHA512")):
         sigs, pubs, dg, hlen, want = workload(curve, 64, tag, hname)
@@ -145,8 +155,6 @@ def test_gpu_ecfsdsa_verify(curve):
 def test_gpu_ecfsdsa_large_batch_properties():
     """2^16 signatures through the chunked host pipeline: tiled reference-made signatures, every 4th corrupted."""
     import libecc_b200
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     curve = "FRP256V1"
     sigs, pubs, dg, hlen, want = workload(curve, 256, 7500)
     reps = 1 << 8

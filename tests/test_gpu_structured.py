@@ -1,6 +1,6 @@
 """The reference's structured key / signature records through the C ABI (SURVEY.md §8f.2) against the UNMODIFIED
-reference (oracle/_ref/libecc_ref.so: ec_structured_*_export_to_buf / _import_from_buf, ec_verify; built in the
-container that has the reference sources and shipped to the GPU box as a prebuilt library)."""
+reference (ec_structured_*_export_to_buf / _import_from_buf, ec_verify through oracle/ref_shim.c; its answers are stored
+under tests/golden/reference/)."""
 import ctypes
 import hashlib
 
@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import libecc_b200
-from common import ALL_CURVES, ORDER, PRIME, oracle_smul, random_scalars, ref_lib, rng
+from common import ALL_CURVES, ORDER, PRIME, oracle_smul, random_scalars, ref_lib, reference_answer, rng
 
 pytestmark = pytest.mark.gpu
 
@@ -25,6 +25,7 @@ def _p(a):
     return np.ascontiguousarray(a).ctypes.data_as(ctypes.c_void_p)
 
 
+@reference_answer
 def ref_keygen(curve, priv: bytes):
     ref = ref_lib()
     prec, pubrec = np.zeros(255, np.uint8), np.zeros(255, np.uint8)
@@ -34,6 +35,7 @@ def ref_keygen(curve, priv: bytes):
     return rc, prec[: pl.value].copy(), pubrec[: ql.value].copy()
 
 
+@reference_answer
 def ref_pub_import(curve, rec):
     ref = ref_lib()
     plen = ALL_CURVES[curve][1]
@@ -44,6 +46,7 @@ def ref_pub_import(curve, rec):
     return rc, aff, inf.value
 
 
+@reference_answer
 def ref_verify(curve, hash_name, sig_rec, pub_rec, msg: bytes):
     ref = ref_lib()
     sig_rec, pub_rec = np.ascontiguousarray(sig_rec), np.ascontiguousarray(pub_rec)
@@ -56,8 +59,6 @@ HASH = {"SHA256": hashlib.sha256, "SHA384": hashlib.sha384, "SHA512": hashlib.sh
 
 @pytest.mark.parametrize("curve", list(ALL_CURVES))
 def test_structured_records_against_reference(curve):
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     cid, plen, qlen = ALL_CURVES[curve]
     q, p = ORDER[curve], PRIME[curve]
     eng = engine(curve)

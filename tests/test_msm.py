@@ -10,12 +10,13 @@ import os
 import numpy as np
 import pytest
 
-from common import ALL_CURVES, ORDER, hostsim_lib, ref_lib, rng, _buf
+from common import ALL_CURVES, ORDER, hostsim_lib, ref_lib, reference_answer, rng, _buf
 from test_ecfsdsa import workload
 
 SEED = bytes(range(7, 39))
 
 
+@reference_answer
 def ref_batch_all(curve, hash_name, sigs, pubs, msgs):
     """The reference's ec_verify_batch(..., ECFSDSA, ...) on the same batch: 0 / -1."""
     ref = ref_lib()
@@ -69,8 +70,6 @@ def test_signed_digit_recoding(c):
                                                ("SECP384R1", "SHA384", 5), ("SECP521R1", "SHA512", 6),
                                                ("SECP224R1", "SHA256", 3), ("SECP192R1", "SHA512", 9)])
 def test_host_algorithm_against_reference(curve, hash_name, c):
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     sigs, pubs, dg, hlen, want = workload(curve, 28, 8900, hash_name)
     good = np.flatnonzero(want == 0)
     ok, stats = host_msm(curve, c, sigs[good], pubs[good], dg[good], hlen)
@@ -94,9 +93,6 @@ def test_host_algorithm_against_reference(curve, hash_name, c):
 def test_host_algorithm_and_reference_batch_entry_point():
     """ec_verify_batch(…, ECFSDSA, …) of the unmodified reference and the multi-scalar-multiplication form agree on
     valid and on corrupted batches (different random coefficients, same verdict)."""
-    ref = ref_lib()
-    if ref is None:
-        pytest.skip("compiled reference not available")
     from test_ecfsdsa import ref_sign, HASH
     from common import random_scalars
     curve, hash_name = "FRP256V1", "SHA256"
@@ -125,8 +121,6 @@ def test_work_per_signature():
     """The count DESIGN.md quotes: field products per signature of the bucket method at the window the library picks
     for 2^20 signatures (c = 16) cannot be run on a CPU; at c = 8 and n = 256 the accumulation already shows the shape:
     one mixed addition per non-zero digit."""
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     curve = "FRP256V1"
     sigs, pubs, dg, hlen, want = workload(curve, 64, 9100)
     good = np.flatnonzero(want == 0)
@@ -176,8 +170,6 @@ def test_square_root_of_the_lift():
 @pytest.mark.parametrize("curve,hash_name,c", [("SECP256K1", "SHA256", 5), ("FRP256V1", "SHA256", 4),
                                                ("SECP256R1", "SHA512", 8), ("SECP384R1", "SHA384", 6)])
 def test_host_bip0340_algorithm_against_reference(curve, hash_name, c):
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     import test_bip0340 as tb
     _, plen, qlen = ALL_CURVES[curve]
     sigs, pubs, dg, hlen, want = tb.workload(curve, 28, 9600, hash_name)
@@ -190,23 +182,19 @@ def test_host_bip0340_algorithm_against_reference(curve, hash_name, c):
     rep = np.repeat(good[:3], 12)
     assert host_msm_bip(curve, 2, sigs[rep], pubs[rep], dg[rep], hlen) == (0, 1)
     # the reference's own batch entry point on the same valid batch, and with one corrupted signature
-    ref = ref_lib()
     privs = __import__("common").random_scalars(curve, 10, tag=9700)
     msgs = [b"bip batch %d" % i for i in range(10)]
     s2, p2 = tb.ref_sign(curve, hash_name, privs, msgs)
-    blob, off = tb.pack(msgs)
     d2 = np.stack([tb.challenge(hash_name, s2[i, :plen], p2[i, :plen], msgs[i]) for i in range(10)])
     for scratch in (0, 1):
-        assert ref.ref_bip0340_verify_batch_all(curve.encode(), hash_name.encode(), 10, _buf(s2), _buf(p2), _buf(blob),
-                                                _buf(off), scratch) == 0
+        assert tb.ref_verify_batch_all(curve, hash_name, s2, p2, msgs, scratch) == 0
     assert host_msm_bip(curve, c, s2, p2, d2, d2.shape[1]) == (0, 1)
     s2[4, -1] ^= 1
     # NOTE: only the reference's scratch-pad-free form (_bip0340_verify_batch_no_memory: the same linear combination,
     # summed directly) is the anchor on corrupted batches.  Its Bos-Coster form (with a scratch pad) was observed here to
     # return 0 for a batch whose s_4 is corrupted - ec_verify_bos_coster (sig/sig_algs.c:1052) leaves its loop as soon as
     # the two largest scalars are equal and then multiplies by their difference, 0 - so it is deliberately not asserted.
-    assert ref.ref_bip0340_verify_batch_all(curve.encode(), hash_name.encode(), 10, _buf(s2), _buf(p2), _buf(blob),
-                                            _buf(off), 0) == -1
+    assert tb.ref_verify_batch_all(curve, hash_name, s2, p2, msgs, 0) == -1
     assert (tb.ref_verify(curve, hash_name, s2, p2, msgs) == [0, 0, 0, 0, -1, 0, 0, 0, 0, 0]).all()
     assert host_msm_bip(curve, c, s2, p2, d2, d2.shape[1]) == (0, 0)
 
@@ -223,8 +211,6 @@ def test_host_bip0340_msm_not_on_secp224r1():
 @pytest.mark.parametrize("curve", list(ALL_CURVES))
 def test_gpu_msm_against_reference(curve, monkeypatch):
     import libecc_b200
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     eng = libecc_b200.Engine(curve, comb_window=8)
     sigs, pubs, dg, hlen, want = workload(curve, 96, 9200)
     good = np.flatnonzero(want == 0)
@@ -256,8 +242,6 @@ def test_gpu_msm_full_size_properties(log2n):
     """2^16 and 2^20 signatures (config 3's batch size): reference-made signatures tiled (equal points meet in the
     buckets), accepted as a whole; one flipped bit anywhere sinks the batch; host and device entry points agree."""
     import libecc_b200
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     curve = "FRP256V1"
     sigs, pubs, dg, hlen, want = workload(curve, 512, 9300)
     good = np.flatnonzero(want == 0)
@@ -282,8 +266,6 @@ def test_gpu_msm_full_size_properties(log2n):
 def test_gpu_bip0340_msm_against_reference(curve, monkeypatch):
     import libecc_b200
     import test_bip0340 as tb
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     eng = libecc_b200.Engine(curve, comb_window=8)
     sigs, pubs, dg, hlen, want = tb.workload(curve, 96, 9800)
     good = np.flatnonzero(want == 0)

@@ -1,13 +1,13 @@
 """Pins the oracle port (oracle/ecc_oracle.c) against the reference's own known-answer vectors
 (tests/golden/*.json, extracted by tests/golden/dump_golden.c from the reference's test headers) and against the
-unmodified reference compiled here (oracle/_ref/libecc_ref.so) on seeded random inputs."""
+unmodified reference's results on seeded random inputs (tests/golden/reference/, see common.reference_answer)."""
 import ctypes
 
 import numpy as np
 import pytest
 
 from common import (hx_fit, ALL_CURVES, CURVES, HASHLEN, ORDER, edge_scalars, golden, hx, oracle_lib, oracle_sign, oracle_smul,
-                    oracle_verify, random_scalars, ref_lib, _buf)
+                    oracle_verify, random_scalars, ref_lib, ref_smul, reference_answer, _buf)
 
 
 @pytest.mark.parametrize("curve", ["SECP256R1", "SECP384R1", "SECP521R1", "SECP224R1", "SECP192R1"])
@@ -96,13 +96,10 @@ def test_wycheproof_ecdh_points(curve):
 
 @pytest.mark.parametrize("curve", list(ALL_CURVES))
 def test_oracle_vs_compiled_reference_random_and_edges(curve):
-    ref = ref_lib()
-    if ref is None:
-        pytest.skip("oracle/_ref/libecc_ref.so not built (needs /root/reference)")
     _, plen, qlen = ALL_CURVES[curve]
     sc = np.concatenate([random_scalars(curve, 24, tag=7, below_q=False), edge_scalars(curve)])
     o1, s1 = oracle_smul(curve, sc)
-    o2, s2 = oracle_smul(curve, sc, lib=ref)
+    o2, s2 = ref_smul(curve, sc)
     assert (s1 == s2).all() and (o1 == o2).all()
     # variable base on the finite results, plus two off-curve points
     good = s1 == 0
@@ -112,23 +109,27 @@ def test_oracle_vs_compiled_reference_random_and_edges(curve):
     pts[1, -1] ^= 1
     pts[2, :plen] = 0xFF  # x >= p
     o3, s3 = oracle_smul(curve, sc2, pts)
-    o4, s4 = oracle_smul(curve, sc2, pts, lib=ref)
+    o4, s4 = ref_smul(curve, sc2, pts)
     assert (s3 == s4).all() and (o3 == o4).all()
     assert s3[1] == -1 and s3[2] == -1
 
 
+@reference_answer
+def ref_smul_long_scalars(curve, sc):
+    n, slen = sc.shape
+    out, st = np.zeros((n, 2 * ALL_CURVES[curve][1]), np.uint8), np.zeros(n, np.int8)
+    ref_lib().ref_prj_pt_mul_batch(curve.encode(), n, _buf(sc), slen, None, _buf(out), _buf(st), 4)
+    return out, st
+
+
 def test_oracle_scalars_longer_than_q_match_reference():
-    ref = ref_lib()
-    if ref is None:
-        pytest.skip("needs the compiled reference")
     curve = "SECP256R1"
     rng = np.random.default_rng(5)
     for slen in (40, 64, 72):
         sc = rng.integers(0, 256, size=(4, slen), dtype=np.uint8)
         out1 = np.zeros((4, 64), np.uint8); st1 = np.zeros(4, np.int8)
-        out2 = np.zeros((4, 64), np.uint8); st2 = np.zeros(4, np.int8)
         oracle_lib().ora_prj_pt_mul_batch(curve.encode(), 4, _buf(sc), slen, None, _buf(out1), _buf(st1), 4)
-        ref.ref_prj_pt_mul_batch(curve.encode(), 4, _buf(sc), slen, None, _buf(out2), _buf(st2), 4)
+        out2, st2 = ref_smul_long_scalars(curve, sc)
         assert (out1 == out2).all() and (st1 == st2).all()
         # (k mod q) * G through python ints
         for i in range(4):

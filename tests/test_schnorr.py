@@ -4,13 +4,14 @@ ECOSDSA verification as the reference defines it (src/sig/ecsdsa_common.c:425-60
 with the caller, as in the reference (src/hash).
 
 CPU: the oracle's double-scalar multiplication + this wrapper against the unmodified reference's verdicts on signatures
-the reference made; the host build of the kernel's algorithm against the oracle.  GPU (`-m gpu`): the C ABI."""
+the reference made (its signatures and verdicts are stored under tests/golden/reference/); the host build of the
+kernel's algorithm against the oracle.  GPU (`-m gpu`): the C ABI."""
 import hashlib
 
 import numpy as np
 import pytest
 
-from common import ALL_CURVES, ORDER, PRIME, hostsim_lib, oracle_lib, oracle_smul, random_scalars, ref_lib, rng, _buf
+from common import ALL_CURVES, ORDER, PRIME, hostsim_lib, oracle_lib, oracle_smul, random_scalars, ref_lib, reference_answer, rng, _buf
 
 HASH = {"SHA256": hashlib.sha256, "SHA384": hashlib.sha384, "SHA512": hashlib.sha512, "SHA224": hashlib.sha224}
 
@@ -22,6 +23,7 @@ def pack(msgs):
     return blob, off
 
 
+@reference_answer
 def ref_siglen(curve, alg, hash_name):
     import ctypes
     sl = ctypes.c_uint32()
@@ -29,6 +31,7 @@ def ref_siglen(curve, alg, hash_name):
     return sl.value
 
 
+@reference_answer
 def ref_sign(curve, alg, hash_name, privs, msgs):
     _, plen, qlen = ALL_CURVES[curve]
     n = len(msgs)
@@ -42,6 +45,7 @@ def ref_sign(curve, alg, hash_name, privs, msgs):
     return sigs, pubs
 
 
+@reference_answer
 def ref_verify(curve, alg, hash_name, sigs, pubs, msgs):
     n = sigs.shape[0]
     blob, off = pack(msgs)
@@ -120,8 +124,6 @@ CASES = [("SECP256R1", "ECSDSA", "SHA256"), ("FRP256V1", "ECOSDSA", "SHA256"), (
 
 @pytest.mark.parametrize("curve,alg,hash_name", CASES)
 def test_oracle_and_host_algorithm_against_reference(curve, alg, hash_name):
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     sigs, pubs, msgs, want = workload(curve, alg, hash_name, 24, 9100)
     got = ecsdsa_verify(curve, hash_name, alg == "ECOSDSA", sigs, pubs, msgs, lambda ab, pk: oracle_double_smul(curve, ab, pk))
     assert (got == want).all()
@@ -188,8 +190,6 @@ def test_gpu_double_smul_against_oracle(curve):
 @pytest.mark.parametrize("curve,alg,hash_name", CASES)
 def test_gpu_ecsdsa_verify_against_reference(curve, alg, hash_name):
     import libecc_b200
-    if ref_lib() is None:
-        pytest.skip("compiled reference not available")
     sigs, pubs, msgs, want = workload(curve, alg, hash_name, 96, 9400)
     eng = libecc_b200.Engine(curve, comb_window=10)
     got = ecsdsa_verify(curve, hash_name, alg == "ECOSDSA", sigs, pubs, msgs, eng.double_smul_batch)
